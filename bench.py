@@ -4,6 +4,16 @@
 
     python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
     python bench.py --impl reference --gpus N ...          # the reference's own CPU implementation
+    python bench.py ... --dump-outputs DIR                 # + the outputs of the last timed walk pass / CBOW step
+
+--dump-outputs writes, after the timed steps of the headline workload (rank 0):
+  walk_rows, walk_lens, walk_keys  generate_paths(canonical=True) of the last timed pass for a fixed sample of 8192
+                                   walkers (walk_index: their rows in the group-0-then-group-1 buffer); keys as two
+                                   32-bit words
+  cbow_W_ih, cbow_W_ho             the weights after the last timed step of --algo (W_ih: a fixed row sample,
+                                   cbow_W_ih_rows, when it exceeds 48 MiB)
+  cbow_accuracy                    that step's validation and training accuracy
+All inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 One "step":  CBOW  = one iteration of the reference's training loop (G2Vec.py:262-267): a full-batch
                      optimizer step over all training windows (fwd+bwd+[all-reduce]+update) plus the
@@ -74,7 +84,13 @@ def parse():
     p.add_argument("--strong-workloads", nargs="*", default=["syn50k", "syn20k"])
     p.add_argument("--cpu-sample-windows", type=int, default=16384)
     p.add_argument("--cpu-walk-seconds", type=float, default=8.0)
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the headline workload's last timed walk pass and CBOW step "
+                        "computed as DIR/<name>.npy (rank 0; a fixed, seeded row sample where an array is large)")
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be at least 1 and --warmup at least 0")
+    return a
 
 
 def workload(name):
@@ -152,6 +168,36 @@ class ClockSampler:
             return None
         load = [x for x in sm if x > 0.5 * max(sm)] or sm
         return {"sm_mhz": float(np.median(load)), "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_BYTES = 64 << 20            # --dump-outputs: all arrays together
+DUMP_WALKERS = 8192              # walker rows in the walk sample (float64, L <= 160: at most 10.5 MB)
+DUMP_W_IH_BYTES = 48 << 20       # W_ih rows beyond this are sampled (stress200k: 410 MB)
+
+
+def sample_rows(n, cap, seed=0):
+    """Sorted indices of a fixed, seeded sample of min(n, cap) of n rows (all of them when n <= cap)."""
+    if n <= cap:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.RandomState(seed).choice(n, cap, replace=False))
+
+
+def key_words(keys):
+    """int64 keys -> [n, 2] (high, low) 32-bit words, which float64 holds exactly."""
+    k = np.asarray(keys, dtype=np.int64).view(np.uint64)
+    return np.stack([k >> np.uint64(32), k & np.uint64(0xFFFFFFFF)], axis=1)
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy, integers as float64 (exact below 2^53), floats as float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32 if np.asarray(a).dtype.kind == "f" else np.float64)
+        total += a.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    assert total <= DUMP_BYTES, "--dump-outputs wrote %d bytes" % total
+    print("bench.py: wrote %d arrays (%.1f MB) to %s" % (len(arrays), total / 1e6, out_dir), file=sys.stderr)
 
 
 def synthetic_windows(N, V, L, device, seed=777):
@@ -239,8 +285,9 @@ def run_b200(args):
     launches0 = _capi.launch_count()
 
     # ------------------------------------------------------------------------------------------ one pipeline
-    def pipeline(wl_name, reps_total, hidden=None, want_e2e=False, want_cbow_detail=False, steps=K, warm=W):
-        """Walks -> windows -> CBOW steps for one workload; walkers rank::world, windows of the rank's own walkers."""
+    def pipeline(wl_name, reps_total, hidden=None, want_e2e=False, want_cbow_detail=False, steps=K, warm=W, dump=None):
+        """Walks -> windows -> CBOW steps for one workload; walkers rank::world, windows of the rank's own walkers.
+        `dump` (a dict) receives the outputs of the last timed walk pass and of the last timed step of args.algo."""
         gs, V, D, L, desc = workload(wl_name)
         D = hidden or D
         graphs = [g2v.WalkGraph(rp, col, weights=w) for rp, col, w in gs]
@@ -279,6 +326,12 @@ def run_b200(args):
         wt, _ = timed(walk_pass, steps)
         barrier()
         walk_launches = _capi.launch_count() - l0
+        if dump is not None:
+            # what generate_paths(canonical=True) returned in the last timed pass: sorted rows, lengths, 64-bit keys
+            idx = sample_rows(2 * n_walk, DUMP_WALKERS)
+            sel = torch.from_numpy(idx).to(dev)
+            dump.update(walk_index=idx, walk_rows=all_rows[sel].cpu().numpy(), walk_lens=all_lens[sel].cpu().numpy(),
+                        walk_keys=key_words(all_keys[sel].cpu().numpy()))
         walk_ms = allmax(float(np.mean(wt)))
         res = {"V": V, "D": D, "L": L, "desc": desc, "walk_ms": walk_ms, "walk_visit_order_ms": allmax(float(np.mean(vt))),
                "visits": visits, "walk_launches": walk_launches, "n_walk": n_walk, "wbytes": wbytes,
@@ -318,14 +371,31 @@ def run_b200(args):
             model.prepare_csc(tr_d)                    # rank1: transposed incidence of the static training list
             slabs = model.prepare_slabs(tr_d)          # rows, table > L2: gene-slab passes
             model.prepare_slabs(va_d)
-            loop = cbow.DeviceLoop(model, ddist, tr_d, va_d, n_tr_tot, 512, False)
+            # the device skips every step past the loop's step cap, so the cap must exceed the longest run of steps
+            # between two resets (warm-up + timed steps; the 5-step production graphs run at most steps + 10)
+            loop = cbow.DeviceLoop(model, ddist, tr_d, va_d, n_tr_tot, max(512, warm + steps + 10), False)
             loop.attach()
+
+            def snapshot():
+                """The weights and the two accuracies of the last step run (dump)."""
+                loop.fetch(); torch.cuda.synchronize()
+                s = int(loop.ctl_pin[1]) - 1
+                correct = loop.hist_pin[4 * s:4 * s + 4].numpy()
+                rows = sample_rows(V, DUMP_W_IH_BYTES // (4 * D))
+                dump.update(cbow_W_ih=model.W_ih[torch.from_numpy(rows).to(dev)].cpu().numpy(),
+                            cbow_W_ho=model.W_ho.cpu().numpy(),
+                            cbow_accuracy=np.array([correct[2] / max(n_va_tot, 1), correct[3] / max(n_tr_tot, 1)]))
+                if len(rows) < V:
+                    dump["cbow_W_ih_rows"] = rows
+            take = dump is not None and algo == args.algo
             try:
                 timed(lambda *m: loop.one(True, *m), warm, marks=3)
                 barrier()
                 l0 = _capi.launch_count()
                 ct, marks = timed(lambda *m: loop.one(True, *m), steps, marks=3)
                 barrier()
+                if take:
+                    snapshot()
                 r = {"launches": _capi.launch_count() - l0, "eager_ms": allmax(float(np.mean(ct))),
                      "fb_ms": float(np.mean([m[0] for m in marks])),
                      "upd_ms": allmax(float(np.mean([m[1] for m in marks]))),
@@ -340,6 +410,8 @@ def run_b200(args):
                     barrier()
                     gt, _ = timed(g_full.replay, steps)
                     barrier()
+                    if take:
+                        snapshot()
                     r["step_ms"], r["graph"] = allmax(float(np.mean(gt))), True
                     loop.reset()
                     g_prod = loop.capture([False] * 4 + [True])
@@ -363,7 +435,8 @@ def run_b200(args):
 
     # ------------------------------------------------------------------------------------------ headline
     reps_total = args.reps * (world if args.scaling == "weak" else 1)
-    P = pipeline(args.workload, reps_total, want_e2e=not args.no_e2e)
+    outputs = {} if (args.dump_outputs and rank == 0) else None
+    P = pipeline(args.workload, reps_total, want_e2e=not args.no_e2e, dump=outputs)
     V, D, L, desc = P["V"], P["D"], P["L"], P["desc"]
     n_tr_tot, n_va_tot, ltr = P["n_tr"], P["n_va"], P["ltr"]
     rowptr, gene, label = P["windows"]
@@ -452,6 +525,8 @@ def run_b200(args):
                                % (int((ltr * 16 + 9).sum()), r["fb_ms"])}
 
     main = P["measure"](args.algo)
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     main_roofline = roofline_of(args.algo, main)
     alt = "rank1" if args.algo == "rows" else "rows"
     ALT = None

@@ -4,6 +4,7 @@ traffic lookup."""
 import os
 import sys
 import time
+import types
 
 import numpy as np
 import pytest
@@ -38,10 +39,19 @@ def test_counting_adjacency_counts_visits_and_stops_on_budget():
         A[6]
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference script not staged")
+def walk_module():
+    """The reference script when it is staged; otherwise the walk port that tests/golden pins bit-exact to the
+    reference's output (oracle.legacy), behind the reference's signature and its global np.random stream."""
+    if ref_import.available():
+        return ref_import.load()
+    from oracle import legacy
+    return types.SimpleNamespace(generate_pathSet=lambda adjMat, maximumLength, iterations: legacy.generate_pathSet_dense(
+        adjMat, maximumLength, iterations, np.random))
+
+
 def test_reference_walk_is_timed_through_its_own_function():
     from tests import helpers
-    ref = ref_import.load()
+    ref = walk_module()
     rp, col, w = helpers.random_graph(150, 5, seed=4)
     rate, visits, dt = bench.cpu_walk_rate(ref, [(rp, col, w)], 20, 0.5, 1)
     assert visits > 200 and 0.4 < dt < 5 and rate == pytest.approx(visits / dt)
@@ -55,3 +65,14 @@ def test_traffic_lookup_matches_only_the_captured_configuration():
     bench._RUN.update(world=2)
     assert bench.traffic_lookup("cbow_rows_fwdbwd", "syn10k") is None          # captures are single-GPU
     bench._RUN.update(world=1)
+
+
+def test_dump_outputs_sample_is_fixed_and_files_are_float(tmp_path):
+    a = bench.sample_rows(100000, 512)
+    assert len(a) == 512 and (np.diff(a) > 0).all() and (a == bench.sample_rows(100000, 512)).all()
+    assert (bench.sample_rows(300, 512) == np.arange(300)).all()
+    bench.write_outputs(str(tmp_path), {"W": np.ones((3, 2), np.float32), "rows": np.array([[1, 2**31 - 1]], np.int32),
+                                        "keys": bench.key_words(np.array([-1, 5], dtype=np.int64))})
+    W, rows, k = (np.load(str(tmp_path / (n + ".npy"))) for n in ("W", "rows", "keys"))
+    assert W.dtype == np.float32 and rows.dtype == np.float64 and k.dtype == np.float64
+    assert rows.tolist() == [[1, 2**31 - 1]] and k.tolist() == [[2**32 - 1, 2**32 - 1], [0, 5]]
