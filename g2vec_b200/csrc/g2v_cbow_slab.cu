@@ -296,7 +296,7 @@ static int launch_fwd_passes(const int32_t *gene, const uint8_t *label, const in
 template <int VEC>
 static int launch_bwd_passes(const int32_t *gene, int64_t n_win, const SlabLayout &l, int32_t S, const float *W_ho,
                              float *g_ih, cudaStream_t st) {
-    const char *sc = getenv("G2V_CBOW_SLAB_SCATTER");             // "tma" (default) / "red": A/B hook, see profiles/r2
+    const char *sc = getenv("G2V_CBOW_SLAB_SCATTER");             // "red" (default) / "tma": A/B hook, see profiles/r2
     const bool tma = sc ? sc[0] == 't' : kDefaultSlabScatterTma;
     auto kern = tma ? cbow_slab_bwd_kernel<VEC, true> : cbow_slab_bwd_kernel<VEC, false>;
     int grid = 0, rc;

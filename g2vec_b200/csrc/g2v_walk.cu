@@ -553,13 +553,18 @@ walk_pair_kernel(const WalkGraphPtrs g, int32_t V, int32_t L, int32_t Lpad, int3
 }
 
 // ---- graph packing (once per graph) -------------------------------------------------------------
+// flag bit 0: some weight is outside [32768, 65536] (no packed 16+16-bit layout); bit 1: some weight exceeds
+// kQwMax, which the short-row path's 32-bit chunk totals (up to 64 weights) cannot hold
+constexpr uint32_t kQwMax = 1u << 24;
 __global__ void walk_range_kernel(const uint32_t *__restrict__ qw, int64_t E, int32_t *__restrict__ flag) {
-    bool bad = false;
+    bool unpackable = false, too_large = false;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < E; i += (int64_t)gridDim.x * blockDim.x) {
         const uint32_t q = __ldg(qw + i);
-        bad = bad || q < 32768u || q > 65536u;
+        unpackable = unpackable || q < 32768u || q > 65536u;
+        too_large = too_large || q > kQwMax;
     }
-    if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) atomicOr(flag, 1);
+    const bool a = __any_sync(0xffffffffu, unpackable), b = __any_sync(0xffffffffu, too_large);
+    if ((a || b) && (threadIdx.x & 31) == 0) atomicOr(flag, (a ? 1 : 0) | (b ? 2 : 0));
 }
 
 // LAY_E8, step 2: one warp per row copies its edges as {col, qw} pairs; an odd row is followed by a {0, 0} pair
@@ -755,23 +760,22 @@ extern "C" int g2v_walk_prepare(const int32_t *rowptr, const int32_t *col, const
     DeviceProps dp;
     if (device_props(&dp)) return 1;
     cudaStream_t st = (cudaStream_t)stream;
-    int layout = LAY_E8;
-    const char *force = getenv("G2V_WALK_LAYOUT");                // test hook: "e8" / "e4" (e4 only if eligible)
-    if (V <= 65535 && !(force && force[1] == '8')) {
-        int32_t *flag = reinterpret_cast<int32_t *>(workspace) + 8;   // the ticket lives in the first 8 bytes
-        int32_t h = 0;
-        G2V_CUDA_OK(cudaMemsetAsync(flag, 0, sizeof(int32_t), st));
-        if (E > 0) {
-            int64_t blocks = (E + 255) / 256;
-            if (blocks > (int64_t)dp.sm_count * 8) blocks = (int64_t)dp.sm_count * 8;
-            walk_range_kernel<<<(unsigned)blocks, 256, 0, st>>>(qw, E, flag);
-            G2V_CUDA_OK(cudaGetLastError());
-            count_launch();
-        }
-        G2V_CUDA_OK(cudaMemcpyAsync(&h, flag, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        G2V_CUDA_OK(cudaStreamSynchronize(st));                   // setup, once per graph
-        if (h == 0) layout = LAY_E4;
+    // one pass over the weights: the qw <= 2^24 contract, and whether the packed 16+16-bit layout can hold them
+    int32_t *flag = reinterpret_cast<int32_t *>(workspace) + 8;   // the ticket lives in the first 8 bytes
+    int32_t h = 0;
+    G2V_CUDA_OK(cudaMemsetAsync(flag, 0, sizeof(int32_t), st));
+    if (E > 0) {
+        int64_t blocks = (E + 255) / 256;
+        if (blocks > (int64_t)dp.sm_count * 8) blocks = (int64_t)dp.sm_count * 8;
+        walk_range_kernel<<<(unsigned)blocks, 256, 0, st>>>(qw, E, flag);
+        G2V_CUDA_OK(cudaGetLastError());
+        count_launch();
     }
+    G2V_CUDA_OK(cudaMemcpyAsync(&h, flag, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    G2V_CUDA_OK(cudaStreamSynchronize(st));                       // setup, once per graph
+    G2V_REQUIRE((h & 2) == 0, "g2v_walk_prepare: an edge weight exceeds the limit qw <= 2^24 = %u", kQwMax);
+    const char *force = getenv("G2V_WALK_LAYOUT");                // test hook: "e8" / "e4" (e4 only if eligible)
+    const int layout = (V <= 65535 && !(force && force[1] == '8') && (h & 1) == 0) ? LAY_E4 : LAY_E8;
     // pads / overhang read as weight-0 (E8) or are overwritten with sentinels (E4): zero the whole buffer first
     G2V_CUDA_OK(cudaMemsetAsync(edges, 0, packed_edge_bytes(V, E), st));
     walk_pack_rows_kernel<<<1, 1024, 0, st>>>(rowptr, V, layout == LAY_E4 ? 4 : 2, reinterpret_cast<int2 *>(rows));

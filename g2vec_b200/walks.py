@@ -24,11 +24,25 @@ def _to_dev(a, dtype, device):
     return torch.from_numpy(a).to(device=device, dtype=dtype, non_blocking=True)
 
 
+def _check_qw(qw):
+    """Integer weights must satisfy qw <= 2^24 (include/g2vec_b200.h): the sampler sums up to 64 of them in 32 bits.
+    int32 storage holds the uint32 bits, so a negative entry is a weight >= 2^31."""
+    if isinstance(qw, torch.Tensor):
+        top = int((qw.to(torch.int64) & 0xFFFFFFFF).max()) if qw.numel() else 0
+    else:
+        a = np.asarray(qw)
+        top = int((a.astype(np.int64) & 0xFFFFFFFF).max()) if a.size else 0
+    if top > _graph.Q_MAX:
+        raise ValueError("integer edge weight %d exceeds the limit qw <= 2^24 = %d" % (top, _graph.Q_MAX))
+
+
 class WalkGraph:
     """One group's directed weighted graph resident in HBM as CSR
     (rowptr int32 [V+1], col int32 [E] ascending per row, qw uint32 [E] stored as int32 bits)."""
 
     def __init__(self, rowptr, col, weights=None, qw=None, device=None):
+        if qw is not None:
+            _check_qw(qw)
         device = _dev(device)
         if qw is None:
             if weights is None:
@@ -56,7 +70,7 @@ class WalkGraph:
         lib = _capi.load()
         self._ws = torch.zeros(max(int(lib.g2v_walk_workspace_bytes()), 64), dtype=torch.uint8, device=device)
         # packed layouts, built once per graph by g2v_walk_prepare: rows = {begin, end} pairs, edges = {col, qw}
-        # pairs (layout 1) or 16+16-bit words, two neighbours per 8-byte load (layout 2: V <= 65536 and weights in
+        # pairs (layout 1) or 16+16-bit words, two neighbours per 8-byte load (layout 2: V <= 65535 and weights in
         # the |PCC| range [0.5, 1])
         import ctypes
         rb, eb = ctypes.c_size_t(0), ctypes.c_size_t(0)

@@ -54,7 +54,8 @@ int64_t g2v_launch_count(void);
  *
  *   rowptr [V+1], col [E] (ascending inside a row = dense row order), qw [E]: CSR of the
  *     group's directed adjacency (rows = out-edges, G2Vec.py:390) with weights quantised to
- *     integers, 1 <= qw <= 2^24  (q = rint(|PCC| * 2^16)).
+ *     integers, 1 <= qw <= 2^24  (q = rint(|PCC| * 2^16)).  g2v_walk_prepare (and so g2v_walk_host) rejects a
+ *     weight above 2^24 with an error; g2v_walk_launch does not check it.
  *   L: --lenPath, the maximum number of NODES of a path (G2Vec.py:331).  1 <= L <= 4096, and the
  *     per-CTA path + visited-set buffers must fit shared memory: always true for L <= 1365, and
  *     for any L <= 4096 while V <= ~90k (bitmap visited set); otherwise the call fails with a message.
@@ -76,7 +77,7 @@ int g2v_walk_launch(const int32_t *rowptr, const int32_t *col, const uint32_t *q
  *   rows  [V]  int32 pairs {begin, end} of each node's out-edges                (g2v_walk_packed_bytes: rows_bytes)
  *   edges      layout 1: uint32 pairs {col, qw}, rows starting at even indices: one 16-byte load brings two
  *              neighbours per lane;
- *              layout 2: uint32 col | (qw - 32768) << 16 [E] -- chosen when V <= 65536 and every
+ *              layout 2: uint32 col | (qw - 32768) << 16 [E] -- chosen when V <= 65535 and every
  *              32768 <= qw <= 65536 (weights |PCC| in [0.5, 1], G2Vec.py:389): one 8-byte load brings two
  *              neighbours per lane                                              (edges_bytes covers both)
  * and returns the layout chosen through *layout_out (a host int; the call synchronises the stream once).

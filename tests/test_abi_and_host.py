@@ -41,6 +41,16 @@ def test_no_cpu_fallback_calls_fail_loudly():
     assert rc != 0 and len(lib.g2v_last_error()) > 0
 
 
+def test_walk_graph_refuses_integer_weights_above_2_to_the_24():
+    """The sampler sums up to 64 weights of a row chunk in 32 bits, so qw <= 2^24 (include/g2vec_b200.h); WalkGraph
+    checks it before touching a device.  int32 storage of the uint32 bits: -1 is 2^32 - 1."""
+    import g2vec_b200
+    rp, col = np.array([0, 2, 2, 2], np.int32), np.array([1, 2], np.int32)
+    for q in (np.array([2**24 + 1, 40000], np.uint32), np.array([40000, -1], np.int32)):
+        with pytest.raises(ValueError, match="2\\^24"):
+            g2vec_b200.WalkGraph(rp, col, qw=q)
+
+
 def test_product_never_imports_the_oracle():
     pkg = os.path.join(ROOT, "g2vec_b200")
     for dirpath, _, files in os.walk(pkg):

@@ -189,7 +189,7 @@ def test_every_layout_and_visited_set_is_bit_exact(g2v, monkeypatch, layout, vis
         n = len(rp) - 1
         want, wl = oracle.walks(rp, col, q, L, 77, 1, 0, reps * n)
         g = g2v.WalkGraph(rp, col, qw=q)
-        packable = q.min() >= 32768 and q.max() <= 65536          # |PCC| in [0.5, 1] and V <= 65536
+        packable = q.min() >= 32768 and q.max() <= 65536          # |PCC| in [0.5, 1] and V <= 65535
         assert g.layout == (2 if (packable and layout != "e8") else 1)
         nodes, lens = g2v.generate_paths(g, L, reps, seed=77, group=1, plain_csr=(layout == "csr"))
         torch.cuda.synchronize()
