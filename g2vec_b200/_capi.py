@@ -63,6 +63,14 @@ SIGNATURES = {
     "g2v_paths_set_select": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp]),
     "g2v_paths_set_emit": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _i64, _i64, _vp, _vp, _vp, _vp,
                                           _vp, _vp]),
+    "g2v_kmeans_workspace_bytes": (ctypes.c_size_t, [_i32, _i32, _i32]),
+    "g2v_kmeans_center": (ctypes.c_int, [_vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "g2v_kmeans_dist": (ctypes.c_int, [_vp, _i32, _i32, _vp, _i32, _vp, _vp, _vp]),
+    "g2v_kmeans_lloyd_step": (ctypes.c_int, [_vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "g2v_post_tscores": (ctypes.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
+    "g2v_post_row_norms": (ctypes.c_int, [_vp, _i64, _i32, _vp, _vp]),
+    "g2v_fmt_row_bytes": (ctypes.c_int, [_vp, _i64, _i32, _vp, _vp, _vp]),
+    "g2v_fmt_emit": (ctypes.c_int, [_vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp]),
     "g2v_test_l2_rows": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp]),
     "g2v_test_draws": (ctypes.c_int, [_u64, _u64, _i32, _vp, _vp]),
     "g2v_test_curand_draws": (ctypes.c_int, [_u64, _u64, _i32, _vp, _vp]),

@@ -377,7 +377,7 @@ def _dist():
 
 def train_cbow(win_rowptr, win_gene, labels, n_genes, hidden, lr, max_epoch=500, seed=0, optimizer="adam",
                reduce="sum", W_ih0=None, W_ho0=None, split=None, early_stop=True, log=print, return_info=False,
-               eval_train="lazy", algo="rows", batch=0, use_graph=True):
+               eval_train="lazy", algo="rows", batch=0, use_graph=True, device_out=False):
     """Train the modified CBOW on CSR windows and return W_ih (np.float32 [n_genes, hidden]) exactly as
     ``compute_genetovec`` does: the weights after the last step whose validation accuracy did not drop.
 
@@ -392,6 +392,9 @@ def train_cbow(win_rowptr, win_gene, labels, n_genes, hidden, lr, max_epoch=500,
     ``use_graph``: on one GPU with full batch, every step after the first replays a CUDA graph of the step's
     launches (the Adam step size lives on the device, g2v_cbow_adam_tick), so the host only replays, waits
     and applies the early-stop rule.
+
+    ``device_out``: return W_ih as a float32 CUDA tensor [n_genes, hidden] instead of a NumPy copy (the steps
+    after training then run on the device, g2vec_b200.post).
     """
     dist = _dist()
     world, rank = (dist.get_world_size(), dist.get_rank()) if dist else (1, 0)
@@ -430,7 +433,7 @@ def train_cbow(win_rowptr, win_gene, labels, n_genes, hidden, lr, max_epoch=500,
                                           max_epoch, early_stop, log, batch)
     if log:
         log("    Optimization Finish")
-    out = out.cpu().numpy()
+    out = out.detach().clone() if device_out else out.cpu().numpy()
     if return_info:
         return out, {"history": hist, "stop_step": stop, "n_train": n_tr, "n_val": n_va, "model": model,
                      "graph": bool(getattr(model, "loop_used_graph", False)), "exchange": model.exchange() if dist else None}

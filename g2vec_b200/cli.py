@@ -3,7 +3,8 @@
 Same positionals, options, progress banners and output files as /root/reference/G2Vec.py
 (parse_arguments :505-518, main :11-119, writers :127-131,159-165,203-215).  Steps 1, 2, 5, 6, 7 are
 plain Python/NumPy/scikit-learn as in the reference; step 3 runs g2vec_b200.walks on the GPU and
-step 4 g2vec_b200.cbow.  Two documented differences: ``--epoch`` is honoured as the cap on optimizer
+step 4 g2vec_b200.cbow.  With ``--post gpu`` steps 5-7 run on the device (g2vec_b200.post) and write the same files;
+the functions here stay the reference for them.  Two documented differences: ``--epoch`` is honoured as the cap on optimizer
 steps (the reference parses it, :515, and then loops ``range(500)``, :262 -- the default 500 is the
 reference behaviour), and ``--seed`` (default 0) makes runs reproducible (the reference is unseeded).
 """
@@ -32,6 +33,9 @@ def parse_arguments(argv=None):
     p.add_argument('--algo', choices=['rows', 'rank1'], default='rows',
                    help="CBOW kernels: 'rows' = embedding-row gather/scatter (default), 'rank1' = collapsed, "
                         "bit-reproducible trainer; same results to fp32 rounding")
+    p.add_argument('--post', choices=['host', 'gpu'], default='host',
+                   help="steps 5-7 (L-groups, gene scores, vectors file): 'host' = NumPy / scikit-learn (default), "
+                        "'gpu' = on the device from the trained vectors (g2vec_b200.post), same files")
     return p.parse_args(argv)
 
 
@@ -93,7 +97,12 @@ def find_lgroups(mat, gene_names, geneFreq):
     (:172,186-187): the outcome is therefore always good = second remaining cluster, poor = first.  That
     behaviour is reproduced here so the output files match."""
     from sklearn.cluster import KMeans
-    km = KMeans(n_clusters=3, random_state=0).fit(mat).labels_
+    return lgroups_from_clusters(KMeans(n_clusters=3, random_state=0).fit(mat).labels_)
+
+
+def lgroups_from_clusters(km):
+    """Cluster ids 0..2 per gene -> L-groups, as find_lgroups numbers them (shared by --post host and gpu)."""
+    km = np.asarray(km)
     sizes = [int(np.count_nonzero(km == k)) for k in range(3)]
     largest = 0
     for k in (1, 2):
@@ -101,7 +110,7 @@ def find_lgroups(mat, gene_names, geneFreq):
             largest = k
     rest = [k for k in (0, 1, 2) if k != largest]
     poor_c, good_c = rest[0], rest[1]
-    out = np.zeros(mat.shape[0], dtype=np.int32)
+    out = np.zeros(km.shape[0], dtype=np.int32)
     out[km == good_c] = 0
     out[km == poor_c] = 1
     out[km == largest] = 2
@@ -227,11 +236,18 @@ def main(argv=None):
 
     print(">>> 4. Compute distributed representations using modified CBOW")
     mat = cbow.train_cbow(w_rowptr, w_gene, w_label, n_genes, args.sizeHiddenlayer, args.learningRate,
-                          max_epoch=args.epoch, seed=args.seed, log=print, algo=args.algo)   # print is silent off rank 0
+                          max_epoch=args.epoch, seed=args.seed, log=print, algo=args.algo,   # print is silent off rank 0
+                          device_out=args.post == 'gpu')
     genes = data['gene']
     if rank != 0:
         dist.barrier()
         dist.destroy_process_group()
+        return
+    if args.post == 'gpu':
+        _post_gpu(args, data, mat, genes, print)
+        if dist is not None:
+            dist.barrier()
+            dist.destroy_process_group()
         return
 
     print('>>> 5. Find L-groups')
@@ -258,6 +274,26 @@ def main(argv=None):
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def _post_gpu(args, data, mat, genes, print):
+    """Steps 5-7 with --post gpu: mat is the device tensor of the vectors; same banners and files as the host."""
+    import torch
+    from . import post
+    print('>>> 5. Find L-groups')
+    lgroup, _ = post.find_lgroups(mat)
+
+    print(">>> 6. Select biomarkers with gene scores")
+    expr = torch.from_numpy(np.ascontiguousarray(data['expr'], dtype=np.float32)).to(mat.device)
+    biomarkers = post.select_biomarkers(mat, expr, data['label'], lgroup, genes, args.numBiomarker)
+
+    print(">>> 7. Save results")
+    write_biomarkers(args.RESULT_NAME, biomarkers)
+    print('    %s_biomarkers.txt' % args.RESULT_NAME)
+    write_lgroups(args.RESULT_NAME, lgroup, genes)
+    print('    %s_lgroups.txt' % args.RESULT_NAME)
+    post.write_vectors(args.RESULT_NAME, genes, mat)
+    print('    %s_vectors.txt' % args.RESULT_NAME)
 
 
 if __name__ == "__main__":

@@ -297,6 +297,44 @@ int g2v_paths_set_emit(const int32_t *rows, const uint8_t *group, const int32_t 
                        int32_t *gene, uint8_t *label, int32_t *freq, int8_t *code, void *stream);
 
 /* ---------------------------------------------------------------------------------------
+ * After training (csrc/g2v_post.cu): the command line's steps 5-7 on the device (--post gpu, g2vec_b200/post.py).
+ *
+ * Step 5, KMeans(n_clusters=3, random_state=0) as scikit-learn runs it.  X [V*D] row-major float32.
+ * g2v_kmeans_workspace_bytes: device scratch for g2v_kmeans_center and g2v_kmeans_lloyd_step (one buffer serves both).
+ * g2v_kmeans_center: mean [D] = float32 column mean, Xc = X - mean, var [D] (double) = per-feature population
+ *   variance (scikit-learn's tol = 1e-4 * mean(var)).
+ * g2v_kmeans_dist: k-means++ distance pass.  cand_host: HOST array of n_cand (1..8) row ids, read before the call
+ *   returns.  out [n_cand*V]: out[k*V + i] = ||X[i] - X[cand[k]]||^2 as float32 (double accumulation), and
+ *   min(closest[i], .) if closest != NULL.  The draws and the choice stay with the caller.
+ * g2v_kmeans_lloyd_step: labels [V] = closest of the K (1..4) centres [K*D] (ties to the lower index), D <= 1024.
+ *   centres_new != NULL: also centres_new = mean of each cluster's rows (the old centre if the cluster is empty) and
+ *   status [2+2K] doubles = {rows whose label differs from labels_old (all rows if labels_old == NULL), empty clusters,
+ *   count[0..K), ||new_k - old_k||^2 [0..K)}.  Fixed-order reductions, no floating-point atomics: bit-reproducible.
+ *
+ * Step 6: g2v_post_tscores: expr [S*V] sample-major, label [S] (0 good, 1 poor, other = neither) -> t [V] = the
+ *   pooled-variance |t| of cli.tscore (ddof = 1; 0 when a group has < 2 samples or the pooled deviation is 0), in
+ *   double.  g2v_post_row_norms: out [V] = ||X[r]||_2.
+ *
+ * Step 7, the vectors file: line r = prefix bytes [prefix_off[r], prefix_off[r+1]) (prefix_off NULL: none) +
+ *   "\t%.6f" per value of X[r] (byte for byte as Python formats a float) + "\n".
+ * g2v_fmt_row_bytes: row_bytes [rows] = length of each line.
+ * g2v_fmt_emit: writes line r at out + offsets[r] (offsets: the caller's exclusive scan of row_bytes).
+ * ------------------------------------------------------------------------------------- */
+size_t g2v_kmeans_workspace_bytes(int32_t V, int32_t D, int32_t K);
+int g2v_kmeans_center(const float *X, int32_t V, int32_t D, float *Xc, float *mean, double *var, void *workspace,
+                      void *stream);
+int g2v_kmeans_dist(const float *X, int32_t V, int32_t D, const int64_t *cand_host, int32_t n_cand,
+                    const float *closest, float *out, void *stream);
+int g2v_kmeans_lloyd_step(const float *X, int32_t V, int32_t D, int32_t K, const float *centres, float *centres_new,
+                          const int32_t *labels_old, int32_t *labels, double *status, void *workspace, void *stream);
+int g2v_post_tscores(const float *expr, int32_t S, int32_t V, const uint8_t *label, float *t, void *stream);
+int g2v_post_row_norms(const float *X, int64_t V, int32_t D, float *out, void *stream);
+int g2v_fmt_row_bytes(const float *X, int64_t rows, int32_t D, const int64_t *prefix_off, int64_t *row_bytes,
+                      void *stream);
+int g2v_fmt_emit(const float *X, int64_t rows, int32_t D, const char *prefix, const int64_t *prefix_off,
+                 const int64_t *offsets, char *out, void *stream);
+
+/* ---------------------------------------------------------------------------------------
  * Test hooks (used by tests/ only): 64-bit draws 0..n-1 of one walker subsequence from the
  * kernel's own Philox, and the same words from curand's Philox4_32_10 generator
  * (curand_init(seed, subsequence, 0)), to prove the stream is curand-compatible.
